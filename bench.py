@@ -199,6 +199,15 @@ def make_batches(wl, n, pinned=False, device=None, seed=1234, image_dtype=None):
     return out
 
 
+def dump_outputs(out_dir, tensors):
+    """Writes each tensor as out_dir/<name>.npy (float64 stays float64, everything else becomes float32)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in tensors.items():
+        t = t.detach().cpu()
+        np.save(os.path.join(out_dir, name + ".npy"), (t if t.dtype == torch.float64 else t.float()).numpy())
+
+
 def run_ours(args):
     from mmnn_sts_b200 import _lib as L, distributed as D
     from mmnn_sts_b200.losses.GradientBlender import GradientBlender
@@ -221,6 +230,7 @@ def run_ours(args):
     # and halves the host->device bytes; --e2e-fp32 ships the reference collate's fp32 tensors instead)
     e2e_dtype = None if args.e2e_fp32 else torch.float16
     host_batches = make_batches(wl, 2, pinned=True, seed=1234 + 100 * rank, image_dtype=e2e_dtype)
+    last = {} if args.dump_outputs else None     # --dump-outputs: what the latest step handed back to its caller
 
     def step(im, cl, ev, du):
         out = model({"image": im, "clinical": cl})
@@ -230,6 +240,8 @@ def run_ours(args):
         sync()
         opt.step()
         opt.zero_grad(set_to_none=True)
+        if last is not None:
+            last["preds"], last["loss"] = out.detach(), loss.detach()
         return loss
 
     def barrier():
@@ -309,6 +321,9 @@ def run_ours(args):
         ms = timed(args.steps, e2e=False)
         launches = (L.lib().mmnn_launch_count() - launches0) // max(1, args.steps)
         ms_e2e = timed(args.steps, e2e=True)
+        if last is not None:                     # the last timed step's outputs, before the untimed steps below move the weights
+            dumped = {k: v.clone() for k, v in last.items()}
+            dumped["state_dict"] = torch.cat([t.detach().reshape(-1).float() for t in model.state_dict().values() if t.is_floating_point()])
         if ms + ms_e2e < 400.0:                  # short runs: keep the same load going until a few 50 ms samples exist
             timed(int((400.0 - ms - ms_e2e) / max(ms / args.steps, 0.1)) + 1, e2e=False)   # (ms is the max over ranks: same count everywhere)
         cs.mark_end()
@@ -423,6 +438,8 @@ def run_ours(args):
         if extra:
             line["extra"] = extra
         print(json.dumps(line), flush=True)
+        if last is not None:
+            dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -715,7 +732,7 @@ def run_reference(args):
     if rank != 0:
         return
     wl = WORKLOADS[args.workload]
-    steps, warmup = max(1, min(args.steps, 3)), max(1, min(args.warmup, 1))
+    steps, warmup = args.steps, max(1, min(args.warmup, 1))
     cpu = cpu_reference_arm(wl, steps=steps, warmup=warmup, sample_batch=wl["batch"])    # the whole batch of 16: same step as the GPU arm
     world = int(os.environ.get("WORLD_SIZE", str(args.gpus)))
     line = {"impl": "reference", "metric": "train volumes/sec", "value": cpu["value"], "unit": "volumes/s", "n_gpus": world,
@@ -742,7 +759,13 @@ if __name__ == "__main__":
     ap.add_argument("--graph", action="store_true", help="replay the device-resident step as one CUDA graph (static shapes)")
     ap.add_argument("--patients", type=int, default=10000)
     ap.add_argument("--resamples", type=int, default=1000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps of the training run, write what its last timed step returned to DIR as .npy: preds "
+                         "(the [3, B, 2] blended heads), loss, and state_dict (every floating-point tensor of the updated model's "
+                         "state_dict, flattened in key order; 45 MB)")
     a = ap.parse_args()
+    if a.dump_outputs and (a.mode != "train" or a.impl != "ours"):
+        ap.error("--dump-outputs applies to the training run of this build (--mode train --impl ours)")
     if a.warmup < 3 and a.impl == "ours":
         a.warmup = 3
     if a.mode == "inference":

@@ -15,7 +15,9 @@ def _free_port():
 
 
 def _worker(rank, world, port, ret):
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank))
+    # no CUDA in the workers: the host logic runs on the CPU even on a machine with fewer GPUs than ranks
+    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank),
+                      CUDA_VISIBLE_DEVICES="")
     from mmnn_sts_b200 import distributed as D
     r, w, dev = D.init_from_env(backend="gloo")
     assert (r, w) == (rank, world) and dev.type == "cpu"
