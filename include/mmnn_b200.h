@@ -115,6 +115,20 @@ struct CindexArgs;
 int mmnn_cindex_bootstrap(const struct CindexArgs* args /*HOST*/, void* stream);
 int mmnn_sizeof_cindex_args(void);
 
+/* mmnn_gradcam_maps : the attention maps of MultiModalGradCAM (/root/reference/utils/utils.py:253-344) for a whole
+ *                     eval-mode batch in ONE launch, replacing the per-patient, per-class trunk backward: the pooled
+ *                     gradient of the last dense layer's conv2 output is computed in closed form from the trunk output y
+ *                     (norm5 -> ReLU -> average pool -> feature_layer -> output_head), then the reference's map arithmetic
+ *                     (cumulative class re-weighting, cam - min, / max, trilinear align_corners=False up-sampling).
+ *                     maps fp32 [B][C][X][Y][Z].  -3 when the C x trunk-voxel cams do not fit shared memory.
+ *                     GradcamArgs: heads.cu. */
+struct GradcamArgs;
+int mmnn_gradcam_maps(const struct GradcamArgs* args /*HOST*/, void* stream);
+int mmnn_sizeof_gradcam_args(void);
+/* CTAs mmnn_gradcam_maps launches for `args` (each reads its sample's trunk-voxel x 32 activations and signs of y once),
+ * for bandwidth accounting; negative: the code mmnn_gradcam_maps would return.  Launches nothing. */
+long long mmnn_gradcam_ctas(const struct GradcamArgs* args /*HOST*/);
+
 /* mmnn_bce_logits   : nn.BCEWithLogitsLoss(pos_weight) of the classification path (/root/reference/main.py:148-153):
  *                     elementwise loss and dloss/dlogit for all stacked heads in one launch (targets [N][C] reused by
  *                     every head), plus the per-class tp / fp / fn counters of main.py:226-229 (sigmoid > threshold). */

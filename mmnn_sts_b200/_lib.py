@@ -94,6 +94,12 @@ class CindexArgs(C.Structure):
                 ("resample", C.c_void_p), ("N", C.c_int), ("R", C.c_int), ("nranks", C.c_int), ("counts", C.c_void_p)]
 
 
+class GradcamArgs(C.Structure):      # csrc/heads.cu
+    _fields_ = [("act", C.c_void_p), ("y", C.c_void_p), ("gamma5", C.c_void_p), ("rvar5", C.c_void_p), ("Wf", C.c_void_p),
+                ("Wo", C.c_void_p), ("maps", C.c_void_p), ("eps", C.c_float)] + \
+               [(n, C.c_int) for n in ("Ctot", "coff", "B", "C", "F", "d", "h", "w", "X", "Y", "Z")]
+
+
 class PackDesc(C.Structure):
     _fields_ = [("src", C.c_void_p), ("dst", C.c_void_p), ("N", C.c_int), ("NT", C.c_int), ("Cin", C.c_int),
                 ("kbw", C.c_int), ("ntaps", C.c_int), ("mode", C.c_int), ("cin_real", C.c_int), ("f16", C.c_int),
@@ -173,7 +179,12 @@ def _declare(l):
     l.mmnn_cox_nll.restype = I
     l.mmnn_cindex_bootstrap.argtypes = [C.POINTER(CindexArgs), VP]
     l.mmnn_cindex_bootstrap.restype = I
-    for nm, st in (("mmnn_sizeof_mlp_args", MlpArgs), ("mmnn_sizeof_cox_args", CoxArgs), ("mmnn_sizeof_cindex_args", CindexArgs)):
+    l.mmnn_gradcam_maps.argtypes = [C.POINTER(GradcamArgs), VP]
+    l.mmnn_gradcam_maps.restype = I
+    l.mmnn_gradcam_ctas.argtypes = [C.POINTER(GradcamArgs)]
+    l.mmnn_gradcam_ctas.restype = LL
+    for nm, st in (("mmnn_sizeof_mlp_args", MlpArgs), ("mmnn_sizeof_cox_args", CoxArgs), ("mmnn_sizeof_cindex_args", CindexArgs),
+                   ("mmnn_sizeof_gradcam_args", GradcamArgs)):
         getattr(l, nm).restype = I
         assert getattr(l, nm)() == C.sizeof(st), (nm, getattr(l, nm)(), C.sizeof(st))
     l.mmnn_sgd_step.argtypes = [C.POINTER(VP), C.POINTER(VP), C.POINTER(VP), C.POINTER(LL), I, C.c_float, C.c_float, C.c_float, I, VP]

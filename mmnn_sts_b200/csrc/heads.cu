@@ -1,8 +1,12 @@
 // Small latency-bound kernels after the trunk: image feature head (ReLU -> global average pool -> Linear -> Dropout),
-// clinical MLP + fusion heads, Cox partial-likelihood loss, bootstrap concordance index.
+// clinical MLP + fusion heads, Cox partial-likelihood loss, bootstrap concordance index, batched GradCAM maps.
 // References: /root/reference/models/densenet.py:234-247, /root/reference/models/mlp.py:19-51,
 // /root/reference/models/multimodal.py:51-80, /root/reference/losses/losses.py:6-9 (pycox CoxPHLoss),
-// /root/reference/main.py:106-123 (lifelines concordance_index).
+// /root/reference/main.py:106-123 (lifelines concordance_index), /root/reference/utils/utils.py:253-344 (GradCAM).
+#include <algorithm>
+#include <climits>
+#include <mutex>
+
 #include "common.cuh"
 #include "prof.h"
 
@@ -501,6 +505,163 @@ __global__ void __launch_bounds__(32) cindex_bootstrap_kernel(const __grid_const
   }
 }
 
+// ---------------------------------------------------------------------------------------------- GradCAM attention maps
+// Batched replacement of MultiModalGradCAM.attentionMaps (/root/reference/utils/utils.py:293-344) for an eval-mode model.
+// The hooked layer is the last conv2 of the last dense block: its 32 output channels are channels [coff, coff + 32) of
+// the block buffer, and they reach the outputs only through norm5 (eval: a fixed affine map) -> ReLU -> global average
+// pool -> feature_layer -> output_head.  So the pooled gradient GradCAM reads has a closed form (no trunk backward):
+//   alpha[b][c][k] = (sum_f Wo[c][f] Wf[f][k']) * gamma5[k'] / sqrt(rvar5[k'] + eps) * count_v(y[b][v][k'] > 0) / V^2,
+// k' = coff + k.  Then the reference's map arithmetic: the activations are re-weighted IN PLACE class after class (class c
+// sees alpha[0] * .. * alpha[c]), cam = channel mean, cam -= min, cam /= max (a constant cam gives NaN, as there), and
+// F.interpolate(mode='trilinear', align_corners=False) to the volume size.  The cam stays 3-D: unlike the reference's
+// .squeeze(), a trunk dimension of size 1 is fine.
+// One launch: CTA (chunk, b) rebuilds sample b's C normalised cams in shared memory (V*32 activations + V*32 signs of y),
+// then streams its range of the [C][X][Y] output rows, Z contiguous floats each.  Every reduction runs in a fixed order.
+struct GradcamArgs {
+  const bf16* act;       // last dense block buffer, storage dtype (fp16 / bf16 per kActF16), [B*V][Ctot]
+  const float* y;        // trunk output (norm5 output) fp32 NDHWC [B*V][Ctot]
+  const float* gamma5;   // norm5.weight        [Ctot]
+  const float* rvar5;    // norm5.running_var   [Ctot]
+  const float* Wf;       // feature_layer.weight [F][Ctot]
+  const float* Wo;       // output_head.weight   [C][2F] (image features first)
+  float* maps;           // [B][C][X][Y][Z]
+  float eps;
+  int Ctot, coff;
+  int B, C, F;
+  int d, h, w;           // trunk dims
+  int X, Y, Z;           // map dims
+};
+constexpr int GC_CH = 32;          // growth rate: channels of the hooked conv
+constexpr int GC_THREADS = 256;
+constexpr size_t GC_SMEM_MAX = 200 * 1024;
+
+__device__ __forceinline__ float gc_act(const bf16* p) {
+  if constexpr (kActF16) return __half2float(*reinterpret_cast<const __half*>(p));
+  else return __bfloat162float(*p);
+}
+
+// min / max that return NaN when either operand is NaN (torch.min / torch.max semantics; fminf / fmaxf skip NaN)
+__device__ __forceinline__ float gc_nanmin(float a, float b) { return (a != a || a < b) ? a : b; }
+__device__ __forceinline__ float gc_nanmax(float a, float b) { return (a != a || a > b) ? a : b; }
+
+// PyTorch's trilinear source index (align_corners=False, size given): src = max(scale (dst + 0.5) - 0.5, 0)
+struct GcLerp { int i0, i1; float l0, l1; };
+__device__ __forceinline__ GcLerp gc_lerp(int dst, float scale, int in) {
+  const float src = fmaxf(scale * ((float)dst + 0.5f) - 0.5f, 0.f);
+  GcLerp r;
+  r.i0 = (int)src;
+  r.i1 = r.i0 + (r.i0 < in - 1 ? 1 : 0);
+  r.l1 = src - (float)r.i0;
+  r.l0 = 1.f - r.l1;
+  return r;
+}
+
+template <bool VEC>
+__global__ void __launch_bounds__(GC_THREADS) gradcam_maps_kernel(const __grid_constant__ GradcamArgs p, int rows_per_cta) {
+  extern __shared__ float gc_smem[];
+  const int C = p.C, V = p.d * p.h * p.w, b = blockIdx.y, tid = threadIdx.y * blockDim.x + threadIdx.x;
+  const int nthr = blockDim.x * blockDim.y, lane = tid & 31, warp = tid >> 5, nwarps = nthr >> 5;
+  float* s_cam = gc_smem;                        // [C][V]
+  float* s_alpha = s_cam + (size_t)C * V;        // [C][32]
+  float* s_line = s_alpha + C * GC_CH;           // [blockDim.y][w]
+  int* s_cnt = reinterpret_cast<int*>(s_line + blockDim.y * p.w);   // [32]
+  const size_t row0 = (size_t)b * V;
+
+  // 1. per-channel positive counts of y (exact integers), the head weights A[c][k] * norm5 scale
+  if (tid < GC_CH) s_cnt[tid] = 0;
+  __syncthreads();
+  {
+    int cnt = 0;                                 // nthr % 32 == 0: this thread always sees channel k = lane
+    for (int i = tid; i < V * GC_CH; i += nthr) cnt += p.y[(row0 + i / GC_CH) * p.Ctot + p.coff + lane] > 0.f ? 1 : 0;
+    if (cnt) atomicAdd(&s_cnt[lane], cnt);
+  }
+  for (int i = tid; i < C * GC_CH; i += nthr) {
+    const int c = i / GC_CH, k = i - c * GC_CH, kk = p.coff + k;
+    float a = 0.f;
+    for (int f = 0; f < p.F; ++f) a = fmaf(p.Wo[(size_t)c * 2 * p.F + f], p.Wf[(size_t)f * p.Ctot + kk], a);
+    s_alpha[i] = a * (p.gamma5[kk] / sqrtf(p.rvar5[kk] + p.eps));
+  }
+  __syncthreads();
+  const float v2 = (float)V * (float)V;
+  for (int i = tid; i < C * GC_CH; i += nthr) s_alpha[i] = s_alpha[i] * ((float)s_cnt[i % GC_CH] / v2);
+  __syncthreads();
+
+  // 2. cams: weighted[k] *= alpha[c][k] class after class (the reference's in-place quirk), cam[c][v] = mean_k weighted[k]
+  for (int v = tid; v < V; v += nthr) {
+    const bf16* a = p.act + (row0 + v) * p.Ctot + p.coff;
+    float wk[GC_CH];
+#pragma unroll
+    for (int k = 0; k < GC_CH; ++k) wk[k] = gc_act(a + k);
+    for (int c = 0; c < C; ++c) {
+      float s = 0.f;
+#pragma unroll
+      for (int k = 0; k < GC_CH; ++k) { wk[k] *= s_alpha[c * GC_CH + k]; s += wk[k]; }
+      s_cam[(size_t)c * V + v] = s / (float)GC_CH;
+    }
+  }
+  __syncthreads();
+
+  // 3. cam -= min; cam /= max (one warp per class, fixed reduction order).  NaN propagates as in torch.min / torch.max: a
+  // cam holding a NaN (a non-finite activation) normalises to all-NaN, like the reference's.
+  for (int c = warp; c < C; c += nwarps) {
+    float* cam = s_cam + (size_t)c * V;
+    float mn = INFINITY, mx = -INFINITY;
+    for (int v = lane; v < V; v += 32) { mn = gc_nanmin(mn, cam[v]); mx = gc_nanmax(mx, cam[v]); }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      mn = gc_nanmin(mn, __shfl_xor_sync(0xffffffffu, mn, o));
+      mx = gc_nanmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+    }
+    const float range = mx - mn;                 // == max(cam - min): x -> fl(x - mn) is monotonic
+    for (int v = lane; v < V; v += 32) cam[v] = (cam[v] - mn) / range;
+  }
+  __syncthreads();
+
+  // 4. trilinear up-sampling of rows [r0, r1) of the flattened [C][X][Y] rows.  Row r is owned by the threads with
+  // threadIdx.y == r % blockDim.y (one warp holds whole rows): they first blend the row's line over (x, y) --
+  // line[j] = lerp_x lerp_y cam[c][.][.][j], j < w -- then write Z outputs, each a lerp of two line entries.
+  const int XY = p.X * p.Y, total = C * XY;
+  const int r0 = blockIdx.x * rows_per_cta, r1 = min(total, r0 + rows_per_cta);
+  const float sx = (float)p.d / (float)p.X, sy = (float)p.h / (float)p.Y, sz = (float)p.w / (float)p.Z;
+  float* line = s_line + threadIdx.y * p.w;
+  float* out_b = p.maps + (size_t)b * total * p.Z;
+  const int nz = VEC ? p.Z / 4 : p.Z;
+  for (int base = r0; base < r1; base += blockDim.y) {
+    const int r = base + threadIdx.y;
+    const bool active = r < r1;
+    if (active) {
+      const int c = r / XY, xy = r - c * XY, x = xy / p.Y, yy = xy - x * p.Y;
+      const GcLerp lx = gc_lerp(x, sx, p.d), ly = gc_lerp(yy, sy, p.h);
+      const float* cc = s_cam + (size_t)c * V;
+      const float* p00 = cc + ((size_t)lx.i0 * p.h + ly.i0) * p.w;
+      const float* p01 = cc + ((size_t)lx.i0 * p.h + ly.i1) * p.w;
+      const float* p10 = cc + ((size_t)lx.i1 * p.h + ly.i0) * p.w;
+      const float* p11 = cc + ((size_t)lx.i1 * p.h + ly.i1) * p.w;
+      for (int j = threadIdx.x; j < p.w; j += blockDim.x)
+        line[j] = lx.l0 * (ly.l0 * p00[j] + ly.l1 * p01[j]) + lx.l1 * (ly.l0 * p10[j] + ly.l1 * p11[j]);
+    }
+    __syncwarp();
+    if (active) {
+      float* orow = out_b + (size_t)r * p.Z;
+      for (int q = threadIdx.x; q < nz; q += blockDim.x) {
+        if constexpr (VEC) {
+          float o[4];
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            const GcLerp lz = gc_lerp(4 * q + j, sz, p.w);
+            o[j] = lz.l0 * line[lz.i0] + lz.l1 * line[lz.i1];
+          }
+          __stcs(reinterpret_cast<float4*>(orow) + q, make_float4(o[0], o[1], o[2], o[3]));
+        } else {
+          const GcLerp lz = gc_lerp(q, sz, p.w);
+          __stcs(orow + q, lz.l0 * line[lz.i0] + lz.l1 * line[lz.i1]);
+        }
+      }
+    }
+    __syncwarp();
+  }
+}
+
 }  // namespace mmnn_heads
 using namespace mmnn_heads;
 
@@ -581,6 +742,84 @@ int mmnn_cox_nll(const CoxArgs* a, void* stream) {
   return 0;
 }
 int mmnn_sizeof_cox_args() { return (int)sizeof(CoxArgs); }
+
+}  // extern "C"
+
+namespace {
+struct GcLaunch { bool vec; dim3 grid, block; size_t smem; int rows_per_cta; };
+constexpr int GC_MAX_DEVICES = 64;
+struct GcVariantCache { size_t smem = 0, smem_attr = 0; int per_sm = 0; };   // last occupancy query; largest smem attribute set
+struct GcDeviceCache { int sms = 0; GcVariantCache variant[2]; };
+GcDeviceCache g_gc_cache[GC_MAX_DEVICES];
+std::mutex g_gc_cache_mutex;
+
+// Launch shape of mmnn_gradcam_maps; 0 or the error code it returns.
+int gradcam_launch_config(const GradcamArgs* a, GcLaunch* L) {
+  if (a->B < 1 || a->B > 65535 || a->C < 1 || a->F < 1 || a->d < 1 || a->h < 1 || a->w < 1 || a->X < 1 || a->Y < 1 ||
+      a->Z < 1 || a->coff < 0 || a->coff + GC_CH > a->Ctot)
+    return -2;
+  const long long V = (long long)a->d * a->h * a->w, rows = (long long)a->C * a->X * a->Y;
+  if (rows > INT_MAX / 2 || V * GC_CH > INT_MAX / 2) return -2;
+  L->vec = a->Z % 4 == 0 && ((uintptr_t)a->maps & 15) == 0;
+  const int nz = L->vec ? a->Z / 4 : a->Z;
+  int bx = 1;
+  while (bx < nz && bx < 32) bx <<= 1;           // threads along Z: a power of two <= 32, so a warp holds whole rows
+  L->block = dim3(bx, GC_THREADS / bx);
+  L->smem = ((size_t)a->C * V + (size_t)a->C * GC_CH + (size_t)L->block.y * a->w + GC_CH) * sizeof(float);
+  if (L->smem > GC_SMEM_MAX) return -3;
+  // >= 2 full waves: CTAs resident per SM x SMs x 2, split evenly over the samples.  The device queries (SM count, the
+  // dynamic shared memory attribute, occupancy) run once per (device, variant, shared memory size), not per batch.
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return (int)e;
+  if (dev < 0 || dev >= GC_MAX_DEVICES) return -2;
+  std::lock_guard<std::mutex> lock(g_gc_cache_mutex);
+  GcDeviceCache& dc = g_gc_cache[dev];
+  if (dc.sms == 0 && (e = cudaDeviceGetAttribute(&dc.sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return (int)e;
+  GcVariantCache& vc = dc.variant[L->vec ? 1 : 0];
+  if (vc.smem != L->smem) {
+    auto kern = L->vec ? gradcam_maps_kernel<true> : gradcam_maps_kernel<false>;
+    if (L->smem > vc.smem_attr) {
+      if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L->smem)) != cudaSuccess) return (int)e;
+      vc.smem_attr = L->smem;
+    }
+    int per_sm = 0;
+    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, GC_THREADS, L->smem)) != cudaSuccess) return (int)e;
+    vc.per_sm = per_sm > 0 ? per_sm : 1;
+    vc.smem = L->smem;
+  }
+  const int sms = dc.sms, per_sm = vc.per_sm;
+  const long long target = 2LL * sms * per_sm;
+  const long long chunks = std::min<long long>(rows, (target + a->B - 1) / a->B);
+  L->rows_per_cta = (int)((rows + chunks - 1) / chunks);
+  L->grid = dim3((unsigned)((rows + L->rows_per_cta - 1) / L->rows_per_cta), (unsigned)a->B);
+  return 0;
+}
+}  // namespace
+
+extern "C" {
+
+// Batched GradCAM maps (MultiModalGradCAM.attentionMaps, /root/reference/utils/utils.py:293-344, for every sample of an
+// eval-mode forward at once).  Shared memory: C*V cams + C*32 weights + one line of w floats per row in flight; -3 when
+// that exceeds GC_SMEM_MAX, -2 for inconsistent sizes.
+int mmnn_gradcam_maps(const GradcamArgs* a, void* stream) {
+  GcLaunch L;
+  const int rc = gradcam_launch_config(a, &L);
+  if (rc != 0) return rc;
+  mmnn::ProfScope ps_(mmnn::PC_HEADS, (cudaStream_t)stream, 1);
+  if (L.vec) gradcam_maps_kernel<true><<<L.grid, L.block, L.smem, (cudaStream_t)stream>>>(*a, L.rows_per_cta);
+  else gradcam_maps_kernel<false><<<L.grid, L.block, L.smem, (cudaStream_t)stream>>>(*a, L.rows_per_cta);
+  LAUNCH_RET();
+  return 0;
+}
+// CTAs mmnn_gradcam_maps launches for these arguments (each reads its sample's V x 32 activations and signs of y once):
+// the byte count of a bandwidth figure.  Negative: the error code mmnn_gradcam_maps would return.
+long long mmnn_gradcam_ctas(const GradcamArgs* a) {
+  GcLaunch L;
+  const int rc = gradcam_launch_config(a, &L);
+  return rc != 0 ? rc : (long long)L.grid.x * L.grid.y;
+}
+int mmnn_sizeof_gradcam_args() { return (int)sizeof(GradcamArgs); }
 
 int mmnn_cindex_bootstrap(const CindexArgs* a, void* stream) {
   const size_t smem = (size_t)(a->nranks + 1 + a->N) * sizeof(int);

@@ -7,7 +7,8 @@
   train_classification /root/reference/main.py:125-327   (BCE-with-logits 'sum' loss with pos_weight, SGD nesterov + OneCycleLR stepped
                                                           every batch, tp / fp / fn -> per-class F1, validation, best-F1 state)
   inference_survival   /root/reference/main.py:750-887   (forward + bootstrap C-index; idiomatic form: every patient is
-                                                          forwarded ONCE, resamples are index multisets)
+                                                          forwarded ONCE, resamples are index multisets; GradCAM maps
+                                                          batched, utils/utils.py:253-344 -> utils.attention_maps)
 Data arrives as an iterable of batches `({'image': ..., 'clinical': ...}, events, durations)` -- what the reference's
 multimodal_collate_fn_surv yields -- so the file/S3 datasets of the reference stay out of scope.
 """
@@ -21,7 +22,7 @@ from .losses.GradientBlender import GradientBlender
 from .losses.losses import CoxPH
 from .ops import concordance_counts
 from .optim import SGD
-from .utils.utils import surv_criterion
+from .utils.utils import attention_maps, surv_criterion
 
 NUM_CLASSES = 2                 # /root/reference/data/constants.py:95
 NUM_BOOTSTRAP_ITERATIONS = 50   # /root/reference/main.py:61
@@ -246,19 +247,29 @@ def train_classification(model, train_batches, val_batches, args, device, grad_s
 
 
 @torch.no_grad()
-def predict_risks(model, batches, device):
-    """Eval-mode forward of every patient once (batched). Returns (preds [N,C], events [N,C], durations [N,C])."""
+def predict_risks(model, batches, device, gradcam=None):
+    """Eval-mode forward of every patient once (batched). Returns (preds [N,C], events [N,C], durations [N,C]).
+    gradcam: optional callable(batch_index, maps).  Each batch then goes through utils.attention_maps (the same forward
+    plus ONE map kernel) and the callable receives that batch's maps [B, C, X, Y, Z] on the device -- the batched form of
+    the reference's per-patient GradCAM loop (/root/reference/main.py:750-887).  Maps are not kept here (at 10 000
+    patients of 128x128x64 they would be 80 GB): the callable writes or reduces them.  The predictions are the same
+    bits either way."""
     model = model.to(device).eval()
     preds, ev, du = [], [], []
-    for batch in batches:
+    for i, batch in enumerate(batches):
         inputs, events, durations = _to_device(batch, device)
-        out = model(inputs)
+        if gradcam is None:
+            out = model(inputs)
+        else:
+            out, maps = attention_maps(model, inputs)
+            gradcam(i, maps)
         preds.append(out[0] if out.dim() == 3 else out); ev.append(events); du.append(durations)
     return torch.cat(preds), torch.cat(ev), torch.cat(du)
 
 
-def inference_survival(model, batches, device, bootstrap=True, num_resamples=NUM_BOOTSTRAP_ITERATIONS, seed=None):
-    preds, events, durations = predict_risks(model, batches, device)
+def inference_survival(model, batches, device, bootstrap=True, num_resamples=NUM_BOOTSTRAP_ITERATIONS, seed=None, gradcam=None):
+    """Risks of every patient, then the C-indices (bootstrap: per-resample, mean, std).  gradcam: see predict_risks."""
+    preds, events, durations = predict_risks(model, batches, device, gradcam=gradcam)
     n = preds.shape[0]
     if not bootstrap:
         return getCIndices(preds, events, durations), preds

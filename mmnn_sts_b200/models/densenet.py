@@ -105,6 +105,7 @@ class Backbone(nn.Sequential):
         self._workspaces = {}
         self.injected_dropmask = None  # tests: [num_layers, B, growth] keep-mask / (1-p)
         self.grad_group_hook = None    # data parallel: callable(backbone, flat_grad) run right after backward is enqueued
+        self._last_forward = None
 
     # ---- C-ABI plumbing
     def _get_plan(self):
@@ -186,6 +187,9 @@ class Backbone(nn.Sequential):
                                           mask.data_ptr() if mask is not None else None, ws.tensor.data_ptr(),
                                           out.data_ptr(), int(self.training), stream)
         L.check(rc, "mmnn_encoder_forward")
+        # (workspace, input shape, trunk dims, fp32 output) of the most recent forward in ANY autograd mode: the batched
+        # attention maps (utils.attention_maps) read it right after a no-grad forward, on the same stream
+        self._last_forward = (ws, (B, cin, X, Y, Z), (dims[0], dims[1], dims[2]), out)
         ws.busy = bool(track)                  # a backward pass will read this workspace
         if ws.busy:
             self._last_ws, self._last_xshape, self._last_out_dims = ws, (B, cin, X, Y, Z), (dims[0], dims[1], dims[2])

@@ -244,3 +244,50 @@ def concordance_counts(event_times, predicted_scores, event_observed, resample_i
     with torch.cuda.device(dev):
         L.check(L.lib().mmnn_cindex_bootstrap(C.byref(a), _stream()), "mmnn_cindex_bootstrap")
     return counts
+
+
+GRADCAM_CHANNELS = 32     # output channels of the hooked conv (the dense layers' growth rate)
+
+
+def gradcam_args(act, y, trunk_dims, norm5_weight, norm5_running_var, eps, feature_weight, head_weight, size):
+    """(GradcamArgs, maps, tensors the struct points to) for mmnn_gradcam_maps; see gradcam_maps."""
+    for t, what in ((act, "gradcam activations"), (y, "gradcam trunk output")):
+        _require_cuda(t, what)
+    d, h, w = (int(v) for v in trunk_dims)
+    X, Y, Z = (int(v) for v in size)
+    M, ctot = act.shape
+    V = d * h * w
+    Fn, Cn = feature_weight.shape[0], head_weight.shape[0]
+    if (M % V or y.numel() != M * ctot or y.dtype != torch.float32 or not y.is_contiguous() or act.stride(1) != 1
+            or act.stride(0) != ctot or tuple(feature_weight.shape) != (Fn, ctot) or tuple(head_weight.shape) != (Cn, 2 * Fn)
+            or norm5_weight.numel() != ctot or norm5_running_var.numel() != ctot or ctot < GRADCAM_CHANNELS):
+        raise ValueError("gradcam_maps: inconsistent shapes")
+    act_dtype = torch.float16 if L.lib().mmnn_act_is_fp16() else torch.bfloat16
+    if act.dtype != act_dtype:
+        raise ValueError(f"gradcam_maps: activations must be in the library's storage dtype {act_dtype}, got {act.dtype}")
+    B = M // V
+    dev = y.device
+    f32 = [t.detach().to(device=dev, dtype=torch.float32).contiguous()
+           for t in (norm5_weight, norm5_running_var, feature_weight, head_weight)]
+    maps = torch.empty((B, Cn, X, Y, Z), dtype=torch.float32, device=dev)
+    a = L.GradcamArgs(_p(act), _p(y), _p(f32[0]), _p(f32[1]), _p(f32[2]), _p(f32[3]), _p(maps), float(eps),
+                      ctot, ctot - GRADCAM_CHANNELS, B, Cn, Fn, d, h, w, X, Y, Z)
+    return a, maps, (act, y, f32)
+
+
+def gradcam_maps(act, y, trunk_dims, norm5_weight, norm5_running_var, eps, feature_weight, head_weight, size):
+    """Batched GradCAM maps of the last dense layer's conv2 in ONE launch (mmnn_gradcam_maps, csrc/heads.cu).
+    act: the last dense block's buffer [B*V, Ctot] in the activation storage dtype (its last 32 channels are the conv's
+    output); y: the trunk's fp32 output (norm5 output, NDHWC) with B*V*Ctot elements; trunk_dims (d, h, w);
+    feature_weight [F, Ctot]; head_weight [C, 2F] (image features first); size (X, Y, Z).
+    Returns fp32 maps [B, C, X, Y, Z].  ValueError when the shapes disagree or the cams do not fit shared memory."""
+    a, maps, _ = gradcam_args(act, y, trunk_dims, norm5_weight, norm5_running_var, eps, feature_weight, head_weight, size)
+    with torch.cuda.device(y.device):
+        rc = L.lib().mmnn_gradcam_maps(C.byref(a), _stream())
+    if rc == -3:
+        raise ValueError(f"gradcam_maps: {a.C} classes x {a.d * a.h * a.w} trunk voxels of cams do not fit the kernel's "
+                         "shared memory")
+    if rc == -2:
+        raise ValueError("gradcam_maps: unsupported sizes")
+    L.check(rc, "mmnn_gradcam_maps")
+    return maps

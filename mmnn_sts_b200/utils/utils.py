@@ -120,3 +120,44 @@ class MultiModalGradCAM(nn.Module):
                 raise AssertionError('attention maps are computed one volume at a time: call with batch size 1')
             maps.append(F.interpolate(cam[None, None], volume_shape, mode='trilinear').squeeze())
         return maps
+
+
+def attention_maps(model, x):
+    """GradCAM attention maps of a whole batch: (outputs, maps [B, num_classes, X, Y, Z]) on the device.
+
+    Batched replacement of the reference's per-patient GradCAM (/root/reference/utils/utils.py:253-344, called per patient
+    from /root/reference/main.py:750-887): the same maps as MultiModalGradCAM.attentionMaps, for any batch size and
+    without a trunk backward.  The pooled gradient of the hooked conv (last conv2 of the last dense block) has a closed
+    form in eval mode -- its output reaches the logits only through norm5 (a fixed affine map), ReLU, the average pool,
+    feature_layer and output_head -- so ONE kernel launch (mmnn_gradcam_maps) rebuilds every sample's cams from the
+    forward's workspace and writes the up-sampled maps.
+
+    `model` is a MultiModalModel (DenseNet121 or TinyDensenet trunk) in eval mode; `x` the {'image', 'clinical'} dict on
+    its CUDA device.  One forward runs under torch.no_grad(), then the kernel is enqueued on the same stream: that order is
+    what keeps the next forward from overwriting the workspace the kernel reads.  The reference's semantics are kept: class
+    c is weighted by the pooled gradients of classes 0..c multiplied together, cam = (cam - min) / max (a constant cam
+    gives NaN), trilinear up-sampling with align_corners=False.  Deliberate differences: a trunk dimension of size 1 works
+    (the reference's .squeeze() breaks on it), and a blended model gives the maps of the multimodal head outputs[0] (the
+    head predict_risks reports; the reference's class raises on it because outputs[0, c] is not a scalar there).
+    Raises ValueError in train mode (batch statistics and dropout break the closed form) and MMNNLibraryError for CPU
+    tensors."""
+    from .. import _lib as L
+    from ..models.densenet import Backbone
+    from ..ops import GRADCAM_CHANNELS, gradcam_maps
+    if model.training:
+        raise ValueError("attention_maps needs an eval-mode model (call model.eval()): batch statistics and dropout "
+                         "break the closed-form pooled gradient")
+    image = x["image"]
+    if not image.is_cuda:
+        raise L.MMNNLibraryError("attention_maps: mmnn_sts_b200 has no CPU path (got a CPU image tensor)")
+    bb = model.gradcam_layer
+    if not isinstance(bb, Backbone) or bb._cfg[3] != GRADCAM_CHANNELS:
+        raise ValueError("attention_maps needs a DenseNet trunk with growth rate %d" % GRADCAM_CHANNELS)
+    with torch.no_grad():
+        outputs = model(x)
+    ws, xshape, dims, y = bb._last_forward
+    act, _ = bb.block_buffer_views(ws, xshape, len(bb._cfg[1]) - 1)
+    feats = model.image_model.model.features.feature_layer
+    maps = gradcam_maps(act, y, dims, bb.norm5.weight, bb.norm5.running_var, bb.norm5.eps, feats.weight,
+                        model.output_head.weight, xshape[2:])
+    return outputs, maps
