@@ -192,6 +192,7 @@ int mmnn_sizeof_aug_intensity(void);
  *                       on different streams of one device must not overlap (MMNN_RN_WGRAD16=0 selects the variant without it).
  * mmnn_rn_bn_coeffs   : nn.BatchNorm3d coefficient table coef fp32 [4][C] = scale, shift, mean, rstd from the batch statistics
  *                       (training: also the running-statistics update, momentum, unbiased variance) or the running ones.
+ *                       C outside 1..64: -2, and nothing is written.
  * mmnn_rn_bn_act      : y = [relu](raw * scale + shift [+ res (res_mode 1) | + res * scale2 + shift2 (res_mode 2)]), then
  *                       nn.Dropout(drop_p) (:156-163) from a counter hash of (seed, element) or an injected uint8 keep-mask.
  * mmnn_rn_act_bwd_reduce / mmnn_rn_bn_bwd_apply : backward of that pass: dz = dy * [y > 0] * post_scale; sums fp64 [3][C] =

@@ -1894,9 +1894,12 @@ int mmnn_rn_conv_wgrad(const RnConvGeom* g, int x_is_f32, const void* x, const v
 int mmnn_rn_bn_coeffs(const double* stats, double count, const float* gamma, const float* beta, float* rmean, float* rvar,
                       long long* nbt, float eps, float momentum, int training, int C, float* coef, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
+  // reject before the launch: the kernel's single 64-thread block would otherwise update the running statistics of the
+  // first 64 channels and num_batches_tracked before the caller learns the call failed
+  if (C < 1 || C > 64) return -2;
   ProfScope ps(PC_RN_ELTWISE, st);
   rn_bn_coeffs_kernel<<<1, 64, 0, st>>>(stats, count, gamma, beta, rmean, rvar, nbt, eps, momentum, training, C, coef);
-  return C > 64 ? -2 : (int)cudaGetLastError();
+  return (int)cudaGetLastError();
 }
 
 int mmnn_rn_bn_act(const void* raw, const float* coef, int res_mode, const void* res, const float* coef2, void* y,

@@ -312,3 +312,47 @@ def test_clinical_only_mlp_forward(training):
         (out * gw.cuda()).sum().backward(); (ref * gw).sum().backward()
         for k, q in m.named_parameters():
             torch.testing.assert_close(q.grad.cpu(), p[pfx + k].grad, rtol=2e-4, atol=2e-5)
+
+
+def _within(got, ref, tol, what):
+    err = (got.double().cpu() - ref).abs()
+    assert bool((err <= tol).all()), f"{what}: worst excess {float((err - tol).max()):.3e}, max |ref| {float(ref.abs().max()):.3e}"
+
+
+@pytest.mark.parametrize("masked", [False, True])
+@pytest.mark.parametrize("B,Cc,V,F", [(1, 1024, 8, 12), (3, 70, 1, 40), (17, 1024, 27, 12), (2, 64, 4096, 3)])
+def test_gap_linear_vs_float64(B, Cc, V, F, masked):
+    """DenseNet feature head (ops.GapLinearDropout: ReLU -> mean over the volume -> Linear -> dropout mask) against float64
+    autograd of Linear(mean_v relu(x)) * mask: the forward and the gradients of x, W and b at 1e-5 of the sum of the absolute
+    terms (fp32 kernels), the ReLU mask of dx exact.  C = 70 is not a multiple of the 32-lane stride, F = 40 is more features
+    than the block's 8 warps."""
+    from mmnn_sts_b200.ops import GapLinearDropout
+    import torch.nn.functional as Fn
+    g = torch.Generator().manual_seed(B * 1000 + V + F)
+    side = {1: (1, 1, 1), 8: (2, 2, 2), 27: (3, 3, 3), 4096: (16, 16, 16)}[V]
+    x = torch.randn((B, Cc) + side, generator=g)
+    W = torch.randn((F, Cc), generator=g) * 0.05
+    b = torch.randn(F, generator=g) * 0.1
+    mask = (torch.rand((B, F), generator=g) >= 0.3).float() / 0.7 if masked else None
+    if masked:
+        mask[0, 0] = 0.0                                 # at least one zero
+    gout = torch.randn((B, F), generator=g)
+    xd, Wd, bd = (t.cuda().requires_grad_(True) for t in (x, W, b))
+    out = GapLinearDropout.apply(xd, Wd, bd, mask.cuda() if masked else None)
+    (out * gout.cuda()).sum().backward()
+    x64, W64, b64 = (t.double().requires_grad_(True) for t in (x, W, b))
+    m64 = mask.double() if masked else torch.ones((B, F), dtype=torch.float64)
+    pooled = x64.clamp_min(0.0).mean(dim=(2, 3, 4))
+    ref = Fn.linear(pooled, W64, b64) * m64
+    (ref * gout.double()).sum().backward()
+    pooled, m64, g64 = pooled.detach(), m64, gout.double()
+    gm = g64 * m64
+    _within(out.detach(), ref.detach(), 1e-5 * (pooled.abs() @ W64.detach().abs().T + b64.detach().abs()) * m64.abs(), "out")
+    # dx = [x > 0] * (g * mask) W / V: exactly zero where x <= 0
+    dxk = xd.grad.cpu()
+    assert bool((dxk[x <= 0] == 0).all())
+    dx_abs = (gm.abs() @ W64.detach().abs() / V)[:, :, None, None, None].expand_as(x64)
+    pos = x > 0
+    _within(dxk[pos], x64.grad[pos], 1e-5 * dx_abs[pos], "dx")
+    _within(Wd.grad, W64.grad, 1e-5 * (gm.abs().T @ pooled.abs()), "dW")
+    _within(bd.grad, b64.grad, 1e-5 * gm.abs().sum(0), "db")

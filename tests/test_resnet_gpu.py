@@ -91,12 +91,17 @@ def test_conv_kernels_match_torch(cin, cout, k, s, p, dims):
         assert lib.mmnn_rn_conv(C.byref(geom), 1, 0, dy_dev.data_ptr(), w_dev.data_ptr(), dx.data_ptr(), None, None, st) == 0
         ref = xa.grad.permute(0, 2, 3, 4, 1)
         assert (dx.float().cpu() - ref).abs().max() <= 1e-2 * ref.abs().max()
+        dx.copy_(add)                                              # the add aliasing the output: what the model's strided
+        assert lib.mmnn_rn_conv(C.byref(geom), 1, 0, dy_dev.data_ptr(), w_dev.data_ptr(), dx.data_ptr(), dx.data_ptr(), None, st) == 0
+        ref = xa.grad.permute(0, 2, 3, 4, 1) + add.float()        # down-sample blocks do, _dgrad(ud, drawd, dx, out=dx)
+        assert (dx.float().cpu() - ref).abs().max() <= 1e-2 * ref.abs().max()
     torch.cuda.synchronize()
 
 
 def test_fused_downsample_pair_matches_separate_calls():
     """mmnn_rn_conv_fwd_ds / mmnn_rn_conv_dgrad_ds (layer1.0: conv1 64 -> 8 3x3x3 + 1x1x1 down-sample on the same input) against
-    the two separate mmnn_rn_conv calls and against torch."""
+    torch.  Under MMNN_RN_MMA=0 there is no fused kernel: both return -9, and the two separate mmnn_rn_conv calls the model
+    then issues (the data gradient's second one in place) are compared with torch instead."""
     from mmnn_sts_b200 import _lib as L
     lib = L.lib()
     dev = torch.device("cuda", 0)
@@ -113,8 +118,14 @@ def test_fused_downsample_pair_matches_separate_calls():
     sd_ = torch.zeros(16, dtype=torch.float64, device=dev)
     st = torch.cuda.current_stream().cuda_stream
     w1d, wdd = w1.to(dev), wd.to(dev)
-    assert lib.mmnn_rn_conv_fwd_ds(C.byref(geom), x_dev.data_ptr(), w1d.data_ptr(), wdd.data_ptr(), y1.data_ptr(), yd.data_ptr(),
-                                   s1.data_ptr(), sd_.data_ptr(), st) == 0
+    mma = os.environ.get("MMNN_RN_MMA", "1")[:1] != "0"           # csrc/resnet.cu rn_mma_enabled()
+    geom_ds = L.RnConvGeom(N, *dims, 64, *dims, 8, 1, 1, 1, 1, 1, 1, 0, 0, 0)
+    rc = lib.mmnn_rn_conv_fwd_ds(C.byref(geom), x_dev.data_ptr(), w1d.data_ptr(), wdd.data_ptr(), y1.data_ptr(), yd.data_ptr(),
+                                 s1.data_ptr(), sd_.data_ptr(), st)
+    assert rc == (0 if mma else -9)
+    if not mma:
+        assert lib.mmnn_rn_conv(C.byref(geom), 0, 0, x_dev.data_ptr(), w1d.data_ptr(), y1.data_ptr(), None, s1.data_ptr(), st) == 0
+        assert lib.mmnn_rn_conv(C.byref(geom_ds), 0, 0, x_dev.data_ptr(), wdd.data_ptr(), yd.data_ptr(), None, sd_.data_ptr(), st) == 0
     r1 = F.conv3d(x, w1, None, 1, 1).permute(0, 2, 3, 4, 1)
     rd = F.conv3d(x, wd, None, 1, 0).permute(0, 2, 3, 4, 1)
     assert (y1.float().cpu() - r1).abs().max() <= 2e-3 * r1.abs().max()
@@ -130,8 +141,12 @@ def test_fused_downsample_pair_matches_separate_calls():
     (F.conv3d(xa, wd.bfloat16().float(), None, 1, 0) * dyd).sum().backward()
     dx = torch.empty((N,) + dims + (64,), dtype=torch.bfloat16, device=dev)
     to_cl = lambda t: t.permute(0, 2, 3, 4, 1).contiguous().to(dev).bfloat16()
-    assert lib.mmnn_rn_conv_dgrad_ds(C.byref(geom), to_cl(dy1).data_ptr(), w1d.data_ptr(), to_cl(dyd).data_ptr(), wdd.data_ptr(),
-                                     dx.data_ptr(), st) == 0
+    dy1_dev, dyd_dev = to_cl(dy1), to_cl(dyd)
+    rc = lib.mmnn_rn_conv_dgrad_ds(C.byref(geom), dy1_dev.data_ptr(), w1d.data_ptr(), dyd_dev.data_ptr(), wdd.data_ptr(), dx.data_ptr(), st)
+    assert rc == (0 if mma else -9)
+    if not mma:
+        assert lib.mmnn_rn_conv(C.byref(geom), 1, 0, dy1_dev.data_ptr(), w1d.data_ptr(), dx.data_ptr(), None, None, st) == 0
+        assert lib.mmnn_rn_conv(C.byref(geom_ds), 1, 0, dyd_dev.data_ptr(), wdd.data_ptr(), dx.data_ptr(), dx.data_ptr(), None, st) == 0
     ref = xa.grad.permute(0, 2, 3, 4, 1)
     assert (dx.float().cpu() - ref).abs().max() <= 1e-2 * ref.abs().max()
     bad = L.RnConvGeom(N, *dims, 64, *dims, 8, 3, 3, 3, 1, 1, 1, 0, 1, 1)
@@ -158,17 +173,18 @@ def test_eval_forward_matches_reference_golden():
     assert int(m.stem[1].num_batches_tracked) == 0
 
 
-def _train_compare(masks_ncdhw, dropout, batch=BATCH, spatial=SPATIAL, grad_tol=0.2, cos_tol=0.985):
+def _train_compare(masks_ncdhw, dropout, batch=BATCH, spatial=SPATIAL, grad_tol=0.2, cos_tol=0.985, training=True):
     """Tolerances: sigmoid scores 5e-3 abs, loss 1e-3 rel (BASELINE north star), gradients by norm-wise relative error and
     cosine against the fp32 oracle.  The default case (3 x 12x32x24) ends in 2x2x2 voxels per sample: BatchNorm over 24 values
     and a gradient that is constant per sample before it make the backward ill-conditioned, which amplifies the bf16
     rounding of the gradient tensors (measured 0.3 % at fc, 6 % at layer4, 8-16 % below, cosine >= 0.99; a larger volume
-    measures the same, so it is the bf16 gradient storage, not the tiny BatchNorm populations)."""
+    measures the same, so it is the bf16 gradient storage, not the tiny BatchNorm populations).  training=False: the model in
+    .eval() (running statistics, no dropout) against the oracle's eval forward, backward included."""
     dev = torch.device("cuda", 0)
     sd = orn.make_state_dict(7, NUM_CLASSES)
     image, labels = orn.make_batch(11, batch, spatial, NUM_CLASSES)
     pos_weight = torch.linspace(0.5, 3.0, NUM_CLASSES)
-    m = _model(dev, sd).train()
+    m = _model(dev, sd).train(training)
     m.dropout.p = 0.2 if dropout else 0.0
     if dropout:
         m.injected_masks = [k.permute(0, 2, 3, 4, 1).contiguous().to(torch.uint8) for k in masks_ncdhw]
@@ -176,7 +192,7 @@ def _train_compare(masks_ncdhw, dropout, batch=BATCH, spatial=SPATIAL, grad_tol=
     loss = F.binary_cross_entropy_with_logits(out, labels.to(dev), pos_weight=pos_weight.to(dev), reduction="sum")
     loss.backward()
     p = {k: (v.clone().requires_grad_(True) if v.is_floating_point() and "running" not in k else v.clone()) for k, v in sd.items()}
-    ref = orn.resnet_forward(p, image, training=True, masks=masks_ncdhw if dropout else None)
+    ref = orn.resnet_forward(p, image, training=training, masks=masks_ncdhw if dropout else None)
     ref_loss = orn.train_step_loss(ref, labels, pos_weight)
     ref_loss.backward()
     assert (out.detach().cpu() - ref.detach()).abs().max() < 5e-3
@@ -197,10 +213,17 @@ def _train_compare(masks_ncdhw, dropout, batch=BATCH, spatial=SPATIAL, grad_tol=
         worst, worst_cos = max(worst, r), min(worst_cos, cos)
         assert r < grad_tol and cos > cos_tol, (k, r, cos)
     msd = m.state_dict()
-    for k in ("stem.1.running_mean", "stem.1.running_var", "layer2.0.downsample.1.running_var", "layer4.1.conv2.1.running_mean"):
-        torch.testing.assert_close(msd[k].cpu(), p[k], rtol=2e-2, atol=2e-3)
-    assert int(msd["layer3.0.conv1.1.num_batches_tracked"]) == 1
-    print(f"[resnet {tuple(spatial)} dropout={dropout}] worst gradient rel-L2 {worst:.3f}, worst cosine {worst_cos:.4f}")
+    if training:
+        for k in ("stem.1.running_mean", "stem.1.running_var", "layer2.0.downsample.1.running_var", "layer4.1.conv2.1.running_mean"):
+            torch.testing.assert_close(msd[k].cpu(), p[k], rtol=2e-2, atol=2e-3)
+        assert int(msd["layer3.0.conv1.1.num_batches_tracked"]) == 1
+    else:
+        for k in msd:
+            if "running" in k:
+                assert torch.equal(msd[k].cpu(), sd[k]), k
+            elif k.endswith("num_batches_tracked"):
+                assert int(msd[k]) == 0, k
+    print(f"[resnet {tuple(spatial)} training={training} dropout={dropout}] worst gradient rel-L2 {worst:.3f}, worst cosine {worst_cos:.4f}")
     return out.detach().cpu(), loss.item(), named, worst
 
 
@@ -226,6 +249,11 @@ def test_train_step_larger_volume():
     # the forward pass is bit-reproducible and this case measures 0.181 every run -> bound 0.25 / cosine 0.96.
     *_, worst = _train_compare(masks, True, batch=4, spatial=(20, 96, 64), grad_tol=0.25, cos_tol=0.96)
     print(f"worst relative gradient error {worst:.3e}")
+
+
+def test_eval_backward_matches_oracle():
+    # .eval(): BatchNorm from the running statistics (mmnn_rn_bn_bwd_apply eval_mode 1), no dropout, nothing updated
+    _train_compare(None, False, training=False)
 
 
 def test_train_step_with_injected_dropout_masks():
