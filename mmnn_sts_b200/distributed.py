@@ -3,7 +3,9 @@
 The reference has no distributed code (SURVEY.md section 2a).  Semantics chosen so that "B patients per GPU on G GPUs"
 equals the reference accumulating G micro-batches of B patients before one optimizer step (/root/reference/main.py:
 469,478-481): BatchNorm statistics and the Cox risk set stay rank-local, gradients are SUMMED (not averaged).
-There is no data-path collective: the only exchange is the gradient all-reduce (payload 11.3 M fp32 = 45 MB)."""
+There is no data-path collective in training: the only exchange is the gradient all-reduce (payload 11.3 M fp32 = 45 MB).
+Inference (main.inference_survival with a group) gathers the per-rank risks with allgather_varlen and splits the
+bootstrap resamples with split_rows."""
 import os
 
 import torch
@@ -137,3 +139,49 @@ def allgather_rows(t, group=None):
     out = [torch.empty_like(t) for _ in range(dist.get_world_size(group))]
     dist.all_gather(out, t.contiguous(), group=group)
     return torch.cat(out, dim=0)
+
+
+def comm_device(device, group=None):
+    """Device on which a collective of `group` takes tensors that live on `device`: that device under NCCL, the host
+    under any other backend (gloo exchanges host memory)."""
+    return torch.device(device) if dist.get_backend(group) == dist.Backend.NCCL else torch.device("cpu")
+
+
+def split_rows(n, rank, world):
+    """[lo, hi): the contiguous share of `n` rows that `rank` of `world` takes.  Every row goes to exactly one rank; the
+    first n % world ranks take one row more, and when n < world the last ranks take none."""
+    q, r = divmod(n, world)
+    lo = rank * q + min(rank, r)
+    return lo, lo + q + (1 if rank < r else 0)
+
+
+def allgather_varlen(t, group=None):
+    """All-gather of per-rank row blocks whose row counts differ (zero included), concatenated in rank order.
+
+    The ranks first exchange their shapes [rows, *row_shape], then every block is padded to the largest row count,
+    gathered and trimmed.  All ranks pass the same dtype and number of dimensions; the non-empty blocks must agree on the
+    row shape, and a rank with no rows may pass any row shape (it cannot know the others'), e.g. torch.empty(0, 0).
+    A mismatch raises ValueError on every rank.  Under NCCL `t` is a CUDA tensor; under gloo the exchange goes through
+    host memory and the result is moved back to `t`'s device."""
+    if not dist.is_initialized() or dist.get_world_size(group) == 1:
+        return t
+    world = dist.get_world_size(group)
+    dev = comm_device(t.device, group)
+    head = torch.tensor(t.shape, dtype=torch.int64, device=dev)
+    heads = [torch.empty_like(head) for _ in range(world)]
+    dist.all_gather(heads, head, group=group)
+    heads = [h.tolist() for h in heads]
+    counts = [h[0] for h in heads]
+    row_shapes = {tuple(h[1:]) for h in heads if h[0] > 0}
+    if len(row_shapes) > 1:
+        raise ValueError("allgather_varlen: ranks disagree on the row shape: %s" % sorted(row_shapes))
+    m = max(counts)
+    if m == 0:
+        return t
+    row_shape = row_shapes.pop()
+    block = torch.zeros((m,) + row_shape, dtype=t.dtype, device=dev)
+    if counts[dist.get_rank(group)]:
+        block[:t.shape[0]] = t
+    out = [torch.empty_like(block) for _ in range(world)]
+    dist.all_gather(out, block, group=group)
+    return torch.cat([o[:c] for o, c in zip(out, counts)]).to(t.device)

@@ -17,7 +17,9 @@ from types import SimpleNamespace
 
 import numpy as np
 import torch
+import torch.distributed as dist
 
+from . import distributed as D
 from .losses.GradientBlender import GradientBlender
 from .losses.losses import CoxPH
 from .ops import concordance_counts
@@ -64,17 +66,27 @@ def getCIndices(preds, events, durations, num_classes=NUM_CLASSES):
     return out
 
 
-def bootstrap_cindices(preds, events, durations, resample_indices, num_classes=NUM_CLASSES):
-    """Per-resample, per-class C-index [R, C] (NaN where a resample has no admissible pair: the reference skips it,
-    /root/reference/main.py:856-858), plus mean and std (ddof 0) over the kept resamples (:883-887)."""
-    counts = torch.stack([concordance_counts(durations[:, i], preds[:, i], events[:, i], resample_indices)
-                          for i in range(num_classes)], dim=1).cpu().numpy()      # [R, C, 3] int64
+def _resample_counts(preds, events, durations, resample_indices, num_classes=NUM_CLASSES):
+    """int64 [R, C, 3] (correct, tied, pairs) of every resample and class, on the predictions' device."""
+    return torch.stack([concordance_counts(durations[:, i], preds[:, i], events[:, i], resample_indices)
+                        for i in range(num_classes)], dim=1)
+
+
+def bootstrap_from_counts(counts):
+    """Per-resample, per-class C-index [R, C] of int64 counts [R, C, 3] (NaN where a resample has no admissible pair: the
+    reference skips it, /root/reference/main.py:856-858), plus mean and std (ddof 0) over the kept resamples (:883-887)."""
     correct, tied, pairs = counts[..., 0], counts[..., 1], counts[..., 2]
     with np.errstate(divide="ignore", invalid="ignore"):
         c = (correct + tied / 2) / pairs
     c[pairs == 0] = np.nan
     ok = ~np.isnan(c).any(axis=1)
-    return c, c[ok].mean(axis=0), c[ok].std(axis=0), counts
+    return c, c[ok].mean(axis=0), c[ok].std(axis=0)
+
+
+def bootstrap_cindices(preds, events, durations, resample_indices, num_classes=NUM_CLASSES):
+    """bootstrap_from_counts of the resamples' counts: (per-resample [R, C], mean, std, counts [R, C, 3])."""
+    counts = _resample_counts(preds, events, durations, resample_indices, num_classes).cpu().numpy()
+    return bootstrap_from_counts(counts) + (counts,)
 
 
 def _with_last_flag(iterable):
@@ -246,14 +258,57 @@ def train_classification(model, train_batches, val_batches, args, device, grad_s
     return hist
 
 
+def _world(group):
+    return 1 if group is None else dist.get_world_size(group)
+
+
+def _gather_patients(preds, events, durations, patient_ids, group, device):
+    """All ranks' rows of (preds, events, durations) in patient order (rank-major without patient_ids).
+
+    One allgather_varlen of float64 rows [preds | events | durations | id]: exact for fp32 predictions and for integer
+    events, durations and ids below 2**53, and a rank without patients needs to know neither C nor the dtypes.  The
+    predictions come back as float32 (the model's output dtype), events and durations as float64 (concordance_counts
+    counts in float64 anyway)."""
+    if preds:
+        cols = [torch.cat(t).to(torch.float64) for t in (preds, events, durations)]
+        if patient_ids is not None:
+            ids = torch.as_tensor(patient_ids).to(device=device, dtype=torch.float64).flatten()
+            if ids.numel() != cols[0].shape[0]:
+                ids = torch.full((cols[0].shape[0],), -1.0, dtype=torch.float64, device=device)   # fails the check below
+            cols.append(ids[:, None])
+        rows = torch.cat(cols, 1)
+    else:
+        rows = torch.empty((0, 0), dtype=torch.float64, device=device)
+    rows = D.allgather_varlen(rows, group)
+    if rows.shape[0] == 0:
+        raise ValueError("inference: no rank forwarded any patient")
+    C = rows.shape[1] // 3
+    if rows.shape[1] % 3:                                         # the id column: some rank passed patient_ids
+        ids = rows[:, 3 * C]
+        order = torch.argsort(ids, stable=True)
+        if not torch.equal(ids[order], torch.arange(rows.shape[0], dtype=torch.float64, device=rows.device)):
+            raise ValueError("inference: the gathered patient_ids are not a permutation of 0..N-1 (N = %d); every rank "
+                             "passes one global patient index per row it forwards" % rows.shape[0])
+        rows = rows[order]
+    return rows[:, :C].to(torch.float32), rows[:, C:2 * C], rows[:, 2 * C:3 * C]
+
+
 @torch.no_grad()
-def predict_risks(model, batches, device, gradcam=None):
+def predict_risks(model, batches, device, gradcam=None, group=None, patient_ids=None):
     """Eval-mode forward of every patient once (batched). Returns (preds [N,C], events [N,C], durations [N,C]).
     gradcam: optional callable(batch_index, maps).  Each batch then goes through utils.attention_maps (the same forward
     plus ONE map kernel) and the callable receives that batch's maps [B, C, X, Y, Z] on the device -- the batched form of
     the reference's per-patient GradCAM loop (/root/reference/main.py:750-887).  Maps are not kept here (at 10 000
     patients of 128x128x64 they would be 80 GB): the callable writes or reduces them.  The predictions are the same
-    bits either way."""
+    bits either way.
+
+    Data parallel (a torch.distributed `group` of more than one rank; group=None is one process): `batches` is this
+    rank's shard, and each rank forwards only its own patients.  The rows of all ranks are then gathered, so every rank
+    returns the same global tensors: in global patient order when `patient_ids` is given (1-D int64, the global index
+    of each of this rank's rows in iteration order, e.g. distributed.shard_patients(N, rank, world); ValueError unless
+    the gathered ids are a permutation of 0..N-1), otherwise rank-major.  Events and durations come back as float64.
+    A rank may have no batches.  GradCAM maps stay on the rank that computed them: `batch_index` counts this rank's
+    batches, so batch k holds the global patients patient_ids[s:s + B_k], s being the rows of batches 0..k-1."""
     model = model.to(device).eval()
     preds, ev, du = [], [], []
     for i, batch in enumerate(batches):
@@ -264,17 +319,57 @@ def predict_risks(model, batches, device, gradcam=None):
             out, maps = attention_maps(model, inputs)
             gradcam(i, maps)
         preds.append(out[0] if out.dim() == 3 else out); ev.append(events); du.append(durations)
+    if _world(group) > 1:
+        return _gather_patients(preds, ev, du, patient_ids, group, device)
     return torch.cat(preds), torch.cat(ev), torch.cat(du)
 
 
-def inference_survival(model, batches, device, bootstrap=True, num_resamples=NUM_BOOTSTRAP_ITERATIONS, seed=None, gradcam=None):
-    """Risks of every patient, then the C-indices (bootstrap: per-resample, mean, std).  gradcam: see predict_risks."""
-    preds, events, durations = predict_risks(model, batches, device, gradcam=gradcam)
+def _draw_resamples(n, num_resamples, seed):
+    """[R, N] bootstrap resamples of patient indices from RandomState(seed), or the global np.random when seed is None.
+    sklearn.utils.resample(uids) == uids[RandomState.randint(0, n, n)]  (SURVEY.md appendix B.3)."""
+    rng = np.random.RandomState(seed) if seed is not None else np.random
+    return np.stack([rng.randint(0, n, n) for _ in range(num_resamples)])
+
+
+def _broadcast_resamples(n, num_resamples, seed, group, device):
+    """int32 [R, N] bootstrap resample matrix on `device`, the same on every rank: rank 0 draws it (_draw_resamples, as
+    the one-process path of inference_survival does) and broadcasts it."""
+    dev = D.comm_device(device, group)
+    if dist.get_rank(group) == 0:
+        idx = torch.as_tensor(_draw_resamples(n, num_resamples, seed)).to(device=dev, dtype=torch.int32)
+    else:
+        idx = torch.empty((num_resamples, n), dtype=torch.int32, device=dev)
+    dist.broadcast(idx, group_src=0, group=group)
+    return idx.to(device)
+
+
+def _bootstrap_split(preds, events, durations, num_resamples, seed, group):
+    """bootstrap_cindices over the ranks of `group`: each rank counts its split_rows(R) rows of the broadcast resample
+    matrix, and the int64 counts are all-gathered, so every rank summarises the same [R, C, 3] counts as one process."""
+    idx = _broadcast_resamples(preds.shape[0], num_resamples, seed, group, preds.device)
+    lo, hi = D.split_rows(num_resamples, dist.get_rank(group), dist.get_world_size(group))
+    if hi > lo:
+        counts = _resample_counts(preds, events, durations, idx[lo:hi])
+    else:
+        counts = torch.empty((0, NUM_CLASSES, 3), dtype=torch.int64, device=preds.device)
+    return bootstrap_from_counts(D.allgather_varlen(counts, group).cpu().numpy())
+
+
+def inference_survival(model, batches, device, bootstrap=True, num_resamples=NUM_BOOTSTRAP_ITERATIONS, seed=None, gradcam=None,
+                       group=None, patient_ids=None):
+    """Risks of every patient, then the C-indices (bootstrap: per-resample, mean, std).  gradcam, group, patient_ids: see
+    predict_risks.  Under a group of more than one rank every rank returns the same result: the gathered predictions of
+    all patients, and the C-indices one process computes from those predictions.  Rank 0 draws the resamples
+    (RandomState(seed), or the global np.random when seed is None; the other ranks' np.random is not advanced) and the
+    ranks split the counting.  A prediction depends slightly on its batch mates (up to ~1e-4 between batches of 4 and
+    11), so it matches a one-process run over other batches to within rounding, not bit for bit (DESIGN.md section 8)."""
+    preds, events, durations = predict_risks(model, batches, device, gradcam=gradcam, group=group, patient_ids=patient_ids)
     n = preds.shape[0]
     if not bootstrap:
         return getCIndices(preds, events, durations), preds
-    # sklearn.utils.resample(uids) == uids[RandomState.randint(0, n, n)]  (SURVEY.md appendix B.3)
-    rng = np.random.RandomState(seed) if seed is not None else np.random
-    idx = np.stack([rng.randint(0, n, n) for _ in range(num_resamples)])
+    if _world(group) > 1:
+        c, mean, std = _bootstrap_split(preds, events, durations, num_resamples, seed, group)
+        return SimpleNamespace(per_resample=c, mean=mean, std=std, preds=preds)
+    idx = _draw_resamples(n, num_resamples, seed)
     c, mean, std, _ = bootstrap_cindices(preds, events, durations, torch.as_tensor(idx, device=preds.device))
     return SimpleNamespace(per_resample=c, mean=mean, std=std, preds=preds)
