@@ -2,14 +2,18 @@
 
 The reference has no distributed code (SURVEY.md section 2a).  Semantics chosen so that "B patients per GPU on G GPUs"
 equals the reference accumulating G micro-batches of B patients before one optimizer step (/root/reference/main.py:
-469,478-481): BatchNorm statistics and the Cox risk set stay rank-local, gradients are SUMMED (not averaged).
-There is no data-path collective in training: the only exchange is the gradient all-reduce (payload 11.3 M fp32 = 45 MB).
+469,478-481): the batch statistics of a forward and the Cox risk set stay within the micro-batch, gradients are SUMMED
+(not averaged).  Within a step the only data-path exchange is the gradient all-reduce (payload 11.3 M fp32 = 45 MB).
+main.train_survival with a group steps on the global micro-batch count (accumulation_rounds), gives a rank without a
+micro-batch in a round zero gradients (fill_missing_grads), merges the BatchNorm running statistics at every step
+(RunningStatsMerger) and gathers the epoch's rows in global order (allgather_ordered).
 Inference (main.inference_survival with a group) gathers the per-rank risks with allgather_varlen and splits the
 bootstrap resamples with split_rows."""
 import os
 
 import torch
 import torch.distributed as dist
+from torch.nn.modules.batchnorm import _BatchNorm
 
 
 def init_from_env(backend=None):
@@ -31,6 +35,150 @@ def shard_patients(num_patients, rank, world, permutation=None):
     """Rank r takes patients perm[r::world] (SURVEY.md section 8e)."""
     perm = permutation if permutation is not None else torch.arange(num_patients)
     return perm[rank::world]
+
+
+def shard_batches(batches, rank, world):
+    """Rank r's round-robin share batches[r::world] of a sequence of micro-batches: local micro-batch i of rank r is
+    global micro-batch i * world + r, the split main.train_survival expects under a group."""
+    return batches[rank::world]
+
+
+def check_interval(interval, world):
+    """ValueError unless `interval` (micro-batches per optimiser step) is a positive integer multiple of `world`: only
+    then does every round of `interval` global micro-batches give each rank the same number of them."""
+    if interval != int(interval) or int(interval) < 1 or int(interval) % world:
+        raise ValueError("data-parallel training needs 64 / batch_size = %s micro-batches per optimiser step to be an "
+                         "integer multiple of the %d ranks" % (interval, world))
+    return int(interval)
+
+
+def check_round_robin(counts, what="micro-batches"):
+    """ValueError unless `counts` (one per rank) are the sizes of a round-robin split of their sum, as shard_batches
+    makes them."""
+    n, world = sum(counts), len(counts)
+    want = [len(range(r, n, world)) for r in range(world)]
+    if list(counts) != want:
+        raise ValueError("per-rank %s counts %s are not a round-robin split of %d (expected %s): shard with "
+                         "distributed.shard_batches" % (what, list(counts), n, want))
+    return n
+
+
+def accumulation_rounds(counts, interval):
+    """[(lo, hi)]: the global micro-batch ranges of one epoch's optimiser steps, given every rank's local micro-batch
+    count (round-robin shards) and `interval` micro-batches per step.  One process steps after micro-batches
+    hi - 1 of these ranges: every `interval`-th one and the last."""
+    interval = check_interval(interval, len(counts))
+    n = check_round_robin(counts)
+    return [(lo, min(lo + interval, n)) for lo in range(0, n, interval)]
+
+
+def allgather_counts(counts, device, group=None):
+    """Every rank's list of integer counts (same length on every rank): [[rank 0's], [rank 1's], ...]."""
+    dev = comm_device(device, group)
+    t = torch.tensor(counts, dtype=torch.int64, device=dev)
+    out = [torch.empty_like(t) for _ in range(dist.get_world_size(group))]
+    dist.all_gather(out, t, group=group)
+    return [o.tolist() for o in out]
+
+
+def fill_missing_grads(reducer):
+    """Before `reducer(model)` in a round where some rank may have done no backward: every parameter that has a
+    gradient on SOME rank gets one on this rank too, zeros where it has none, so that every rank enters the same
+    collectives in GradientAllReducer.  Costs one all-reduce of a per-parameter int32 flag.
+
+    A module with a flat gradient buffer (the DenseNet trunk) gets its zeros from `pack_flat_grad()`, which backs every
+    parameter's .grad with views of one buffer, so that flat_grad_buffer() is not None on any rank and all of them
+    reduce that module with one collective."""
+    params, group = reducer.params, reducer.group
+    if not params:
+        return
+    has = torch.tensor([p.grad is not None for p in params], dtype=torch.int32, device=comm_device(params[0].device, group))
+    dist.all_reduce(has, op=dist.ReduceOp.MAX, group=group)
+    need = {id(p) for p, h in zip(params, has.tolist()) if h}
+    for m in reducer.flat_modules:
+        if any(id(p) in need for p in m.parameters()):
+            m.pack_flat_grad()
+    for p in params:
+        if p.grad is None and id(p) in need:
+            p.grad = torch.zeros_like(p)
+
+
+class RunningStatsMerger:
+    """BatchNorm running statistics over the ranks of `group` equal to one process forwarding the same global
+    micro-batches in order, with no kernel change.
+
+    A training forward applies r <- a r + m x (a = 1 - m) to each running buffer.  Over a round of n global
+    micro-batches one process ends with r_end = a^n r_start + sum_k m a^(n-1-k) x_k.  Each rank snapshots the buffers
+    before each of its forwards (`before_forward`), recovers d_k = u_after - a u_before = m x_k after it
+    (`after_forward(k)`, k = the micro-batch's position in the round), and accumulates S += a^(n-1-k) d_k in float64 on
+    the device.  `merge()` all-reduces S together with the num_batches_tracked increments and sets r = a^n r_start + S
+    and num_batches_tracked = its value at `begin` + the summed increments.  Between `begin` and `merge` a rank's
+    buffers hold its own local EMA.  Tracks every _BatchNorm with running statistics; `momentum=None` (cumulative
+    average) is refused with ValueError, and `momentum` must be what the module's forward applies."""
+
+    def __init__(self, model, group=None):
+        self.group = group
+        mods = [m for m in model.modules() if isinstance(m, _BatchNorm) and m.track_running_stats]
+        for m in mods:
+            if m.momentum is None:
+                raise ValueError("RunningStatsMerger: a BatchNorm with momentum=None (cumulative moving average) cannot "
+                                 "be merged over ranks")
+        self.stats = [t for m in mods for t in (m.running_mean, m.running_var)]
+        self.counts = [m.num_batches_tracked for m in mods]
+        if not mods:
+            return
+        dev = self.stats[0].device
+        self._numel = sum(t.numel() for t in self.stats)
+        self._decay = torch.cat([torch.full((t.numel(),), 1.0 - m.momentum, dtype=torch.float64)
+                                 for m in mods for t in (m.running_mean, m.running_var)]).to(dev)
+        # fp32 snapshots as views of flat buffers, built once: the copies are single multi-tensor launches (same dtype)
+        # and the float64 arithmetic runs on the flat buffers, so a micro-batch costs a handful of launches
+        self._start, self._before, self._after = (torch.empty(self._numel, dtype=torch.float32, device=dev) for _ in range(3))
+        self._start_v, self._before_v, self._after_v = (self._views(f) for f in (self._start, self._before, self._after))
+        self._acc = torch.zeros(self._numel + len(self.counts), dtype=torch.float64, device=dev)   # [S | increments]
+        self._count_start = torch.empty(len(self.counts), dtype=torch.int64, device=dev)
+        self._n = 0
+
+    def _views(self, flat):
+        out, off = [], 0
+        for t in self.stats:
+            out.append(flat[off:off + t.numel()].view(t.shape))
+            off += t.numel()
+        return out
+
+    def begin(self, n):
+        """Start a round of `n` global micro-batches (every rank calls it, with the same n)."""
+        self._n = n
+        if not self.counts:
+            return
+        torch._foreach_copy_(self._start_v, self.stats)
+        torch.stack(self.counts, out=self._count_start)
+        self._acc.zero_()
+
+    def before_forward(self):
+        if self.counts:
+            torch._foreach_copy_(self._before_v, self.stats)
+
+    def after_forward(self, k):
+        """After the training forward of the round's k-th global micro-batch (0-based)."""
+        if not self.counts:
+            return
+        torch._foreach_copy_(self._after_v, self.stats)
+        d = self._after.double().addcmul_(self._decay, self._before.double(), value=-1.0)     # d_k = m x_k
+        self._acc[:self._numel].addcmul_(self._decay.pow(self._n - 1 - k), d)
+
+    def merge(self):
+        """Set every rank's buffers to the one-process values at the end of the round (a collective)."""
+        if not self.counts:
+            return
+        self._acc[self._numel:] = torch.stack(self.counts) - self._count_start
+        dev = comm_device(self._acc.device, self.group)
+        acc = self._acc.to(dev)
+        dist.all_reduce(acc, op=dist.ReduceOp.SUM, group=self.group)
+        acc = acc.to(self._acc.device)
+        self._after.copy_(self._decay.pow(self._n) * self._start.double() + acc[:self._numel])
+        torch._foreach_copy_(self.stats, self._after_v)
+        torch._foreach_copy_(self.counts, list((self._count_start + acc[self._numel:].to(torch.int64)).unbind()))
 
 
 class GradientAllReducer:
@@ -185,3 +333,15 @@ def allgather_varlen(t, group=None):
     out = [torch.empty_like(block) for _ in range(world)]
     dist.all_gather(out, block, group=group)
     return torch.cat([o[:c] for o, c in zip(out, counts)]).to(t.device)
+
+
+def allgather_ordered(rows, group=None):
+    """allgather_varlen of float64 rows [n, 2 + w] whose first two columns are integer keys (global micro-batch index,
+    row index within it), returned sorted by (micro-batch, row) without the key columns: the rows of round-robin
+    shards in the order one process sees them.  A rank without rows passes torch.empty(0, 0)."""
+    rows = allgather_varlen(rows, group)
+    if rows.shape[0] == 0:
+        return rows
+    rows = rows[torch.argsort(rows[:, 1], stable=True)]
+    rows = rows[torch.argsort(rows[:, 0], stable=True)]
+    return rows[:, 2:]

@@ -109,18 +109,39 @@ def _to_device(batch, device):
     return inputs, events.to(device, non_blocking=True), durations.to(device, non_blocking=True)
 
 
-def train_survival(model, train_batches, val_batches, args, device, grad_sync=None, log=None):
-    """args: lr, momentum, weight_decay, epochs, batch_size, blend, blend_update_interval, num_train (patients).
-    grad_sync: optional callable(model) run right before each optimizer.step (data-parallel gradient all-reduce)."""
-    model = model.to(device)
+def _survival_setup(model, args):
+    """Optimiser, OneCycleLR schedule (ceil(num_train / 64) steps per epoch), blender and the empty history."""
     n_train = args.num_train
-    super_batch_interval = SUPER_BATCH_SIZE / args.batch_size
     steps_per_epoch = n_train // SUPER_BATCH_SIZE if n_train % SUPER_BATCH_SIZE == 0 else 1 + n_train // SUPER_BATCH_SIZE
     optimizer = SGD(model.parameters(), args.lr, momentum=args.momentum, nesterov=True, weight_decay=args.weight_decay)
     scheduler = torch.optim.lr_scheduler.OneCycleLR(optimizer, max_lr=args.lr, steps_per_epoch=steps_per_epoch, epochs=args.epochs)
     blender = GradientBlender(CoxPH, survival=True, surv_criterion=surv_criterion) if args.blend else None
     hist = SimpleNamespace(train_loss=[], val_loss=[], train_c=[], val_c=[], best_loss=math.inf, best_state=None, blender=blender,
                            step_at=[], lr_trace=[], momentum_trace=[], optimizer=optimizer, scheduler=scheduler)
+    return optimizer, scheduler, blender, hist
+
+
+def train_survival(model, train_batches, val_batches, args, device, grad_sync=None, log=None, group=None):
+    """args: lr, momentum, weight_decay, epochs, batch_size, blend, blend_update_interval, num_train (patients).
+    grad_sync: optional callable(model) run right before each optimizer.step (data-parallel gradient all-reduce).
+
+    group: a torch.distributed group of more than one rank trains data-parallel as one process would on all ranks'
+    micro-batches (DESIGN.md section 8).  `train_batches` / `val_batches` are then this rank's round-robin shards
+    (distributed.shard_batches: local micro-batch i of rank r is global micro-batch i * G + r) and must support len();
+    args.num_train is the GLOBAL patient count; 64 / batch_size must be a multiple of G.  train_survival reduces the
+    gradients itself (passing grad_sync too raises ValueError), steps after every 64 global patients and after the last
+    micro-batch, merges the BatchNorm running statistics at every step, and computes the epoch's losses, C-indices,
+    best state and blending-weight update from all ranks' rows in global order, so every rank returns the same hist.
+    group=None, or a group of one rank, is the one-process loop."""
+    if _world(group) > 1:
+        if grad_sync is not None:
+            raise ValueError("train_survival: with a group of several ranks train_survival reduces the gradients itself; "
+                             "do not pass grad_sync")
+        return _train_survival_dp(model, train_batches, val_batches, args, device, log, group)
+    model = model.to(device)
+    n_train = args.num_train
+    super_batch_interval = SUPER_BATCH_SIZE / args.batch_size
+    optimizer, scheduler, blender, hist = _survival_setup(model, args)
     for epoch in range(args.epochs):
         model.train()
         losses, c_pred, c_events, c_durations = [], [], [], []
@@ -176,6 +197,151 @@ def train_survival(model, train_batches, val_batches, args, device, grad_sync=No
                 blender.updateWeights(c_pred, c_events, c_durations, y_pred, y_events, y_durations)
         if log is not None:
             log(f"epoch {epoch + 1}: train loss {hist.train_loss[-1]:.4f} train C {hist.train_c[-1]}")
+    return hist
+
+
+def _len_or_flag(batches):
+    """len(batches); -1 when it has none, -2 for None (exchanged, so that every rank raises on a bad input)."""
+    if batches is None:
+        return -2
+    return len(batches) if hasattr(batches, "__len__") else -1
+
+
+def _keyed_rows(g, preds, events, durations):
+    """float64 rows [g, row, H, preds (H x C), events (C), durations (C)] of one micro-batch (H = 1 for [B, C] preds):
+    exact for fp32 predictions and integer targets below 2**53, and self-describing, so that a rank without rows can
+    still decode what the others gathered."""
+    p = preds.detach()
+    H = p.shape[0] if p.dim() == 3 else 1
+    p = p.permute(1, 0, 2).reshape(p.shape[-2], -1) if p.dim() == 3 else p
+    B = p.shape[0]
+    dev = p.device
+    keys = torch.stack([torch.full((B,), float(g), dtype=torch.float64, device=dev),
+                        torch.arange(B, dtype=torch.float64, device=dev),
+                        torch.full((B,), float(H), dtype=torch.float64, device=dev)], 1)
+    return torch.cat([keys, p.to(torch.float64), events.to(torch.float64).reshape(B, -1),
+                      durations.to(torch.float64).reshape(B, -1)], 1)
+
+
+def _gather_rows(rows, stacked, group, device):
+    """All ranks' _keyed_rows in global order: (preds [H, N, C] if stacked else [N, C] float32, events, durations
+    float64 [N, C])."""
+    rows = torch.cat(rows) if rows else torch.empty((0, 0), dtype=torch.float64, device=device)
+    rows = D.allgather_ordered(rows, group)
+    N = rows.shape[0]
+    if N == 0:
+        raise ValueError("train_survival: no rank has a micro-batch")
+    H = int(rows[0, 0])
+    C = (rows.shape[1] - 1) // (H + 2)
+    preds = rows[:, 1:1 + H * C].to(torch.float32)
+    preds = preds.reshape(N, H, C).permute(1, 0, 2).contiguous() if stacked else preds
+    return preds, rows[:, 1 + H * C:1 + (H + 1) * C], rows[:, 1 + (H + 1) * C:]
+
+
+def _gather_scalars(rows, width, group, device):
+    """All ranks' per-micro-batch scalar rows [g, 0, value...] in global micro-batch order: float64 [N_b, width]."""
+    rows = torch.stack(rows) if rows else torch.empty((0, 0), dtype=torch.float64, device=device)
+    return D.allgather_ordered(rows, group).reshape(-1, width)
+
+
+def _train_survival_dp(model, train_batches, val_batches, args, device, log, group):
+    """train_survival over the ranks of `group` (see there).  The collectives a rank enters depend only on what every
+    rank agrees on (args, the world size and the exchanged per-rank batch counts), never on its own data."""
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    interval = D.check_interval(SUPER_BATCH_SIZE / args.batch_size, world)       # raises before any collective
+    model = model.to(device)
+    n_train = args.num_train
+    optimizer, scheduler, blender, hist = _survival_setup(model, args)
+    merger = D.RunningStatsMerger(model, group)
+    hooks = [(m, m.grad_group_hook) for m in model.modules() if hasattr(m, "grad_group_hook")]   # restored on return
+    reducer = D.GradientAllReducer(model.parameters(), group=group, model=model)
+
+    def loss_of(outputs, events, durations):
+        if args.blend:
+            return blender.computeLoss(outputs, events, durations)
+        loss = surv_criterion(CoxPH, outputs, events, durations, device)
+        return loss, loss
+
+    try:
+        for epoch in range(args.epochs):
+            counts = D.allgather_counts([_len_or_flag(train_batches), _len_or_flag(val_batches)], device, group)
+            if any(c[0] == -1 or c[1] == -1 for c in counts):
+                raise TypeError("train_survival: under a group every rank's train_batches and val_batches must support "
+                                "len() (a list, a DataLoader): the ranks agree on the step schedule before the epoch")
+            if any(c[0] < 0 for c in counts) or len({c[1] == -2 for c in counts}) > 1:
+                raise ValueError("train_survival: every rank passes train_batches, and either every rank or none val_batches")
+            rounds = D.accumulation_rounds([c[0] for c in counts], interval)
+            has_val = counts[0][1] != -2
+            n_val_batches = D.check_round_robin([c[1] for c in counts], "validation micro-batches") if has_val else 0
+            if not rounds:
+                raise ValueError("train_batches has no batch in epoch %d" % (epoch + 1))
+            model.train()
+            it = iter(train_batches)
+            losses, rows = [], []
+            for lo, hi in rounds:
+                merger.begin(hi - lo)
+                for g in range(lo + rank, hi, world):
+                    inputs, events, durations = _to_device(next(it), device)
+                    merger.before_forward()
+                    outputs = model(inputs)
+                    merger.after_forward(g - lo)
+                    loss, _ = loss_of(outputs, events, durations)
+                    if hi - lo == world:
+                        reducer.arm()       # every rank has exactly this one micro-batch: reduce during backward
+                    loss.backward()
+                    losses.append(torch.stack([torch.full_like(loss.detach(), g, dtype=torch.float64),
+                                               torch.zeros((), dtype=torch.float64, device=loss.device), loss.detach().double()]))
+                    rows.append(_keyed_rows(g, outputs, events, durations))
+                D.fill_missing_grads(reducer)
+                reducer(model)
+                merger.merge()
+                optimizer.step()
+                scheduler.step()
+                optimizer.zero_grad(set_to_none=True)
+                hist.step_at.append((epoch, hi - 1))
+                hist.lr_trace.append(optimizer.param_groups[0]["lr"]); hist.momentum_trace.append(optimizer.param_groups[0]["momentum"])
+            c_pred, c_events, c_durations = _gather_rows(rows, args.blend, group, device)
+            if c_events.shape[0] != n_train:
+                raise ValueError("train_survival: the ranks trained %d patients in epoch %d, args.num_train is %d (the "
+                                 "global count)" % (c_events.shape[0], epoch + 1, n_train))
+            train_losses = _gather_scalars(losses, 1, group, device)[:, 0].to(torch.float32)
+            hist.train_c.append(getCIndices(c_pred[0] if args.blend else c_pred, c_events, c_durations))
+            hist.train_loss.append(float(train_losses.sum()) / n_train)
+            if has_val:
+                if n_val_batches == 0:
+                    raise ValueError("val_batches has no batch in epoch %d" % (epoch + 1))
+                model.eval()
+                with torch.no_grad():
+                    vrows, vlosses, i = [], [], -1
+                    for i, batch in enumerate(val_batches):
+                        g = i * world + rank
+                        inputs, events, durations = _to_device(batch, device)
+                        preds = model(inputs)
+                        loss, sel = loss_of(preds, events, durations)
+                        vlosses.append(torch.stack([torch.full_like(loss, g, dtype=torch.float64),
+                                                    torch.zeros((), dtype=torch.float64, device=loss.device),
+                                                    loss.double(), sel.double()]))
+                        vrows.append(_keyed_rows(g, preds, events, durations))
+                    if i + 1 != counts[rank][1]:
+                        raise ValueError("val_batches yielded %d batches, len() said %d" % (i + 1, counts[rank][1]))
+                    y_pred, y_events, y_durations = _gather_rows(vrows, args.blend, group, device)
+                    vl = _gather_scalars(vlosses, 2, group, device).tolist()
+                    vloss = 0.0
+                    for loss, _ in vl:
+                        vloss += loss                      # fp32 values as Python floats, summed in global order
+                    sel = vl[-1][1]                        # the globally last validation micro-batch
+                    hist.val_c.append(getCIndices(y_pred[0] if args.blend else y_pred, y_events, y_durations))
+                    hist.val_loss.append(vloss / max(1, y_events.shape[0]))
+                    if sel < hist.best_loss:
+                        hist.best_loss = sel
+                        hist.best_state = {k: v.detach().clone() for k, v in model.state_dict().items()}
+                if args.blend and (epoch + 1) % args.blend_update_interval == 0:
+                    blender.updateWeights(c_pred, c_events, c_durations, y_pred, y_events, y_durations)
+            if log is not None:
+                log(f"epoch {epoch + 1}: train loss {hist.train_loss[-1]:.4f} train C {hist.train_c[-1]}")
+    finally:
+        for m, h in hooks:
+            m.grad_group_hook = h
     return hist
 
 

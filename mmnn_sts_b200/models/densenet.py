@@ -267,6 +267,26 @@ class Backbone(nn.Sequential):
             off += n
         return flat
 
+    def pack_flat_grad(self):
+        """Make flat_grad_buffer() return a buffer: if it does not, every parameter's .grad becomes a view of one fresh
+        fp32 buffer holding its current gradient (zeros where it has none).  A data-parallel rank that did no backward
+        in an accumulation round then reduces the trunk with the same single collective as the other ranks."""
+        flat = self.flat_grad_buffer()
+        if flat is not None:
+            return flat
+        self._get_plan()
+        params = list(self.parameters())
+        flat = torch.zeros(sum(self._numel), dtype=torch.float32, device=params[0].device)
+        off = 0
+        for p, n in zip(params, self._numel):
+            v = flat[off:off + n].view(p.shape)
+            if p.grad is not None:
+                v.copy_(p.grad)
+            p.grad = v
+            off += n
+        self._flat_grad = flat
+        return flat
+
     def forward(self, x):
         params = tuple(self.parameters())
         if torch.is_grad_enabled() and any(p.requires_grad for p in params):
